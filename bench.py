@@ -50,10 +50,17 @@ METRIC = "residual+Jacobian evals/sec (full LM solves)"
 UNIT = "residual evals/s"
 
 
+def positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError(f"must be >= 1, got {v}")
+    return v
+
+
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=positive_int, default=200, help="timed steps (full LM solves), exactly this many")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", choices=["ours", "reference"], default="ours")
     ap.add_argument("--frames", type=int, default=FRAMES_PER_GPU, help="frames per GPU")
@@ -64,6 +71,7 @@ def parse_args():
     ap.add_argument("--no-config3", action="store_true", help="skip the supplementary 4.8 GB rows (configs[2] and configs[4])")
     ap.add_argument("--no-strong", action="store_true", help="skip the strong-scaling leg (configs[3], 48 GB over the N ranks)")
     ap.add_argument("--strong-frames", type=int, default=1_000_000)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed solve returned as DIR/<name>.npy (rank 0)")
     return ap.parse_args()
 
 
@@ -130,14 +138,14 @@ def cpu_reference_problem(frames, beams):
 
 
 def time_cpu_solve(p, threads, linear_solver):
-    """One full LM solve with the oracle; returns (seconds, residual evaluations, iterations)."""
+    """One full LM solve with the oracle; returns (seconds, residual evaluations, iterations, (pose7, summary, trace))."""
     from oracle import oracle as O
 
     opt = O.default_options(linear_solver=linear_solver, num_threads=threads)
     t0 = time.perf_counter()
-    _, s, _ = O.solve(p, X0, opt)
+    x, s, tr = O.solve(p, X0, opt)
     dt = time.perf_counter() - t0
-    return dt, s.num_residual_evaluations * p.num_residuals(), s.num_iterations
+    return dt, s.num_residual_evaluations * p.num_residuals(), s.num_iterations, (x, s, tr)
 
 
 def pick_threads(p):
@@ -166,16 +174,16 @@ def cpu_baseline(frames, beams, quick=False):
     n = min(frames, CPU_SAMPLE_FRAMES)
     p = cpu_reference_problem(n, beams)
     cores = pick_threads(p)
-    dt1, ev1, iters = time_cpu_solve(p, 1, 0)
+    dt1, ev1, iters, _ = time_cpu_solve(p, 1, 0)
     best = dict(value=ev1 / dt1, cores=1)
     extras = {"ceres_shaped_1_thread": {"value": ev1 / dt1, "unit": UNIT, "cores": 1}}
     if cores > 1:
-        dta, eva, _ = time_cpu_solve(p, cores, 0)
+        dta, eva, _, _ = time_cpu_solve(p, cores, 0)
         extras["ceres_shaped_best_thread_count"] = {"value": eva / dta, "unit": UNIT, "cores": cores}
         if eva / dta > best["value"]:
             best = dict(value=eva / dta, cores=cores)
     if not quick:
-        dts, evs, _ = time_cpu_solve(p, cores, 1)  # most favourable CPU variant: streaming normal equations
+        dts, evs, _, _ = time_cpu_solve(p, cores, 1)  # most favourable CPU variant: streaming normal equations
         extras["streaming_normal_equations_best_thread_count"] = {"value": evs / dts, "unit": UNIT, "cores": cores}
     extras["host_cpus_visible"] = os.cpu_count()
     out = dict(value=best["value"], unit=UNIT, cores=best["cores"], kind="port",
@@ -201,19 +209,21 @@ def run_reference(args):
     # threads: the better of 1 (what the reference uses) and all host threads, decided on the warm-up solves
     rates = {}
     for th in sorted({1, cores}):
-        dt, ev, _ = time_cpu_solve(p, th, 0)
+        dt, ev, _, _ = time_cpu_solve(p, th, 0)
         rates[th] = ev / dt
     cores = max(rates, key=rates.get)
     for _ in range(max(0, args.warmup - len(rates))):
         time_cpu_solve(p, cores, 0)
     t_tot, ev_tot, iters, steps_done = 0.0, 0, 0, 0
     for _ in range(args.steps):
-        dt, ev, iters = time_cpu_solve(p, cores, 0)
+        dt, ev, iters, result = time_cpu_solve(p, cores, 0)
         t_tot += dt
         ev_tot += ev
         steps_done += 1
-        if t_tot > 120.0:  # keep the whole run within a few minutes whatever --steps says
-            break
+    if args.dump_outputs:
+        from oracle import oracle as O
+
+        dump_solve_outputs(args.dump_outputs, *result, O.Iteration)
     value = ev_tot / t_tot
     sample = (f"each step = one full LM solve on the first {n} of {args.frames} frames x {args.beams} points "
               f"({n * args.beams} residuals, {iters} iterations); Ceres-shaped oracle port, evaluation on {cores} threads")
@@ -297,6 +307,22 @@ def solve_row(prob, opt, reps, n_points_total, max_over_ranks, barrier):
     return x, {"ms_per_solve": ms / reps, "sweeps_per_solve": sweeps / reps, "lm_iterations_per_solve": iters / reps,
                "residual_evals_per_s": n_points_total * sweeps / (ms * 1e-3), "lm_iters_per_s": iters / (ms * 1e-3),
                "termination": int(s.termination)}
+
+
+def dump_solve_outputs(out_dir, x, summary, trace, iteration_type):
+    """What a solve returned (Problem.solve, or the oracle's for --impl reference), one float64 .npy per quantity: pose7
+    (T_cl), summary_<field> and trace_<field> (one entry per LM iteration, fields of iteration_type).  The timing
+    (device_ms) and padding fields are left out: they are not results."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"pose7": x}
+    for name, _ in type(summary)._fields_:
+        if name not in ("reserved", "device_ms"):
+            arrays["summary_" + name] = getattr(summary, name)
+    for name, _ in iteration_type._fields_:
+        if name != "reserved":
+            arrays["trace_" + name] = [getattr(t, name) for t in trace]
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def run_ours(args):
@@ -401,7 +427,7 @@ def run_ours(args):
     dev_ms, sweeps, iters, per_step = 0.0, 0, 0, []
     x = X0
     for _ in range(args.steps):
-        x, s, _ = prob.solve(X0, opt)
+        x, s, trace = prob.solve(X0, opt)
         dev_ms += s.device_ms
         per_step.append(s.device_ms)
         sweeps += s.num_sweeps
@@ -409,6 +435,10 @@ def run_ours(args):
     barrier()
     wall_ms = 1e3 * (time.perf_counter() - t0)
     launches = launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        from camlasercalibratool_b200._lib import LmIteration
+
+        dump_solve_outputs(args.dump_outputs, x, s, trace, LmIteration)
     dev_ms = max_over_ranks(dev_ms)
     wall_ms = max_over_ranks(wall_ms)
     value = total_points * sweeps / (dev_ms * 1e-3)
@@ -563,7 +593,7 @@ def run_ours(args):
                     "kernels": "general three-stream kernels (24 B/residual contract row); planar rows separate",
                     "check": check, "strong_scaling": strong, "step_device_ms": step_stats})
         line = {
-            "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
+            "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": len(per_step), "warmup": args.warmup,
             "ms_per_step": dev_ms / args.steps, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
             "dtype": "f64", "data": "synthetic", "config": cfg,
             "lm_iters_per_s": lm_iters_per_s, "sweeps_per_solve": sweeps / args.steps, "lm_iterations_per_solve": iters / args.steps,

@@ -56,15 +56,16 @@ REPO = os.path.dirname(PKG_DIR)
 DROPIN_SRC = os.path.join(PKG_DIR, "host", "LaseCamCalB200.cpp")
 BENCH_SRC = os.path.join(PKG_DIR, "host", "dropin_bench.cpp")
 BENCH_EXE = os.path.join(PKG_DIR, "host", "clc_dropin_bench")
-REFERENCE_INCLUDE = "/root/reference/include"
 
 
 def interface_include_dirs():
-    """Include path of the reference interface: the reference's own include/LaseCamCalCeres.h when the tree is present
-    (build container), else the test stand-in; Eigen itself is not in this image, so its few types come from tests/stubs."""
+    """Include path of the reference interface: the reference's own include/LaseCamCalCeres.h when the environment variable
+    CLC_REFERENCE_INCLUDE names a directory that holds it (a checkout of the reference's include/), else the test stand-in;
+    Eigen itself is not required, its few types come from tests/stubs."""
     dirs = []
-    if os.path.exists(os.path.join(REFERENCE_INCLUDE, "LaseCamCalCeres.h")):
-        dirs.append(REFERENCE_INCLUDE)
+    ref = os.environ.get("CLC_REFERENCE_INCLUDE")
+    if ref and os.path.exists(os.path.join(ref, "LaseCamCalCeres.h")):
+        dirs.append(ref)
     dirs.append(os.path.join(REPO, "tests", "stubs"))
     dirs.append(os.path.join(REPO, "include"))
     return dirs

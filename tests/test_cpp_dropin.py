@@ -15,19 +15,31 @@ def build_driver(out_dir):
 
     _lib.load()
     exe = os.path.join(out_dir, "host_dropin_test")
-    # against the reference's own include/LaseCamCalCeres.h when /root/reference exists (build container), else the stand-in
+    # against the reference's own include/LaseCamCalCeres.h when CLC_REFERENCE_INCLUDE names it, else the stand-in
     subprocess.check_call(_build.cxx_command([os.path.join(ROOT, "tests", "host_dropin_test.cpp"), _build.DROPIN_SRC], exe))
     return exe
 
 
-def test_dropin_compiles_against_the_reference_header_when_present():
+def test_dropin_compiles_against_the_reference_header_when_present(tmp_path, monkeypatch):
     from camlasercalibratool_b200 import _build
 
-    dirs = _build.interface_include_dirs()
-    if os.path.exists("/root/reference/include/LaseCamCalCeres.h"):
-        assert dirs[0] == "/root/reference/include"  # the genuine interface wins over tests/stubs/LaseCamCalCeres.h
-    else:
-        assert dirs[0].endswith(os.path.join("tests", "stubs"))
+    stubs = os.path.join(ROOT, "tests", "stubs")
+    monkeypatch.delenv("CLC_REFERENCE_INCLUDE", raising=False)
+    assert _build.interface_include_dirs()[0] == stubs
+    ref = tmp_path / "include"
+    ref.mkdir()
+    monkeypatch.setenv("CLC_REFERENCE_INCLUDE", str(ref))  # no header there: the stand-in stays
+    assert _build.interface_include_dirs()[0] == stubs
+    # a directory with the interface header wins over tests/stubs/LaseCamCalCeres.h, and the drop-in builds against it; the
+    # probe lives outside that directory, so only the include path can lead it to the marked header
+    with open(os.path.join(stubs, "LaseCamCalCeres.h")) as f:
+        header = f.read()
+    (ref / "LaseCamCalCeres.h").write_text("#define CLC_TEST_REFERENCE_HEADER_USED 1\n" + header)
+    assert _build.interface_include_dirs()[0] == str(ref)
+    probe = tmp_path / "probe.cpp"
+    probe.write_text('#include "LaseCamCalCeres.h"\n#ifndef CLC_TEST_REFERENCE_HEADER_USED\n#error stand-in header used\n#endif\n')
+    for src in (str(probe), _build.DROPIN_SRC):
+        subprocess.check_call(_build.cxx_command([src], str(tmp_path / "obj.o"), extra=("-c",)))
 
 
 def test_bench_driver_builds():
