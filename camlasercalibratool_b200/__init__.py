@@ -21,6 +21,7 @@ from .api import (  # noqa: F401
     launch_count,
     marshal,
     pose7_to_T,
+    problems_from_scans,
     shard_range,
     upload_stats,
 )
@@ -28,4 +29,5 @@ from .api import (  # noqa: F401
 __all__ = [
     "CamLaserCalClosedSolution", "CamLaserCalibration", "LineFittingCeres", "ClcError", "Comm", "Group", "Oberserve", "Problem", "T_to_pose7",
     "comm_unique_id", "default_options", "launch_count", "marshal", "pose7_to_T", "shard_range", "debug_pack", "upload_stats",
+    "problems_from_scans",
 ]

@@ -9,7 +9,7 @@ PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG_DIR, "csrc")
 LIB_PATH = os.path.join(PKG_DIR, "libclc_b200.so")
 SOURCES = ["clc_api.cu", "clc_pack.cpp"]
-HEADERS = ["clc_kernels.cuh", "clc_math.cuh", "clc_lm.cuh", "clc_expand.cuh", "clc_linefit.cuh", "clc_camera.cuh", "clc_upload.inl"]
+HEADERS = ["clc_kernels.cuh", "clc_math.cuh", "clc_lm.cuh", "clc_expand.cuh", "clc_linefit.cuh", "clc_scans.cuh", "clc_camera.cuh", "clc_upload.inl"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-lineinfo", "-std=c++17",

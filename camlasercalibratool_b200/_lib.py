@@ -78,6 +78,27 @@ class CameraDesc(C.Structure):
     ]
 
 
+class ScanDesc(C.Structure):
+    _fields_ = [
+        ("n_scans", C.c_int64),
+        ("n_beams", C.c_int64),
+        ("ranges", C.POINTER(C.c_float)),
+        ("scan_stamp", c_double_p),
+        ("angle_min", C.c_double),
+        ("angle_increment", C.c_double),
+        ("range_min", C.c_double),
+        ("n_poses", C.c_int64),
+        ("pose_stamp", c_double_p),
+        ("pose_wc", c_double_p),
+        ("max_dt", C.c_double),
+        ("line_fit_max_iterations", C.c_int),
+        ("with_edges", C.c_int),
+        ("use_loss", C.c_int),
+        ("cauchy_a", C.c_double),
+        ("device", C.c_int),
+    ]
+
+
 class LmOptions(C.Structure):
     _fields_ = [
         ("max_num_iterations", C.c_int),
@@ -168,6 +189,9 @@ SIGNATURES = {
     "clc_line_fit_points": (C.c_int, [c_double_p, C.c_int64, c_double_p, C.c_int]),
     "clc_scan_segments": (C.c_int, [C.POINTER(C.c_float), C.c_int64, C.c_int64, C.c_double, C.c_double, C.c_double,
                                     C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.c_int]),
+    "clc_problems_create_from_scans": (C.c_int, [C.POINTER(ScanDesc), C.POINTER(_P), C.POINTER(_P), C.POINTER(C.c_int32),
+                                                 c_double_p]),
+    "clc_scan_last_stats": (C.c_int, [C.POINTER(C.c_float), c_int64_p, c_int64_p]),
     "clc_estimate_board_poses": (C.c_int, [C.POINTER(CameraDesc), C.c_int64, c_int64_p, C.POINTER(C.c_int32), C.POINTER(C.c_float),
                                            c_double_p, C.POINTER(C.c_int32), C.c_int]),
     "clc_T_to_pose7": (None, [c_double_p, c_double_p]),

@@ -14,7 +14,7 @@ from dataclasses import dataclass, field
 import numpy as np
 
 from . import _lib
-from ._lib import ClcError, GatherDesc, LmIteration, LmOptions, LmSummary, ProblemDesc, SyntheticDesc, TERMINATION
+from ._lib import ClcError, GatherDesc, LmIteration, LmOptions, LmSummary, ProblemDesc, ScanDesc, SyntheticDesc, TERMINATION
 
 
 def _dp(a):
@@ -497,6 +497,52 @@ class pinned_array:
             self._ptr = None
 
 
+def problems_from_scans(ranges, scan_stamps, angle_min, angle_increment, range_min, pose_stamps, pose_wc, max_dt=0.02,
+                        line_fit_max_iterations=10, with_edges=False, use_loss=True, cauchy_a=0.05, device=-1):
+    """The offline driver's scan loop on the device (clc_problems_create_from_scans, reference main/calibr_offline.cpp:86-155):
+    ranges[n_scans, n_beams] float32 (a pinned_array's array is used as the DMA source), scan_stamps[n_scans],
+    pose_stamps[n_poses], pose_wc[n_poses, 7] = qx qy qz qw x y z of T_wc.  Returns (points_problem, on_line_problem,
+    scan_info[n_scans, 4] int32 = seg_start, seg_end, nearest pose, frame (-1: none), scan_line[n_scans, 2] (NaN where no
+    frame)).  The points problem holds Oberserve::points, the on-line problem Oberserve::points_on_line (+ edge residuals
+    when with_edges)."""
+    L = _lib.load()
+    r = np.asarray(ranges)
+    if r.dtype != np.float32:
+        raise ValueError("ranges must be float32 (sensor_msgs/LaserScan::ranges)")
+    r = np.ascontiguousarray(r)
+    if r.ndim != 2:
+        raise ValueError("ranges must be [n_scans, n_beams]")
+    ts = np.ascontiguousarray(scan_stamps, dtype=np.float64).reshape(-1)
+    if ts.shape[0] != r.shape[0]:
+        raise ValueError("one stamp per scan is needed")
+    tp = np.ascontiguousarray(pose_stamps, dtype=np.float64).reshape(-1)
+    pw = np.ascontiguousarray(pose_wc, dtype=np.float64).reshape(-1, 7)
+    if pw.shape[0] != tp.shape[0]:
+        raise ValueError("one pose per pose stamp is needed")
+    d = ScanDesc()
+    d.n_scans, d.n_beams = r.shape
+    d.ranges = r.ctypes.data_as(C.POINTER(C.c_float))
+    d.scan_stamp = _dp(ts)
+    d.angle_min, d.angle_increment, d.range_min = float(angle_min), float(angle_increment), float(range_min)
+    d.n_poses, d.pose_stamp, d.pose_wc = tp.shape[0], _dp(tp), _dp(pw)
+    d.max_dt, d.line_fit_max_iterations, d.with_edges = float(max_dt), int(line_fit_max_iterations), int(bool(with_edges))
+    d.use_loss, d.cauchy_a, d.device = int(bool(use_loss)), float(cauchy_a), int(device)
+    info = np.empty((r.shape[0], 4), dtype=np.int32)
+    lines = np.empty((r.shape[0], 2))
+    hp, hl = C.c_void_p(), C.c_void_p()
+    _lib.check(L.clc_problems_create_from_scans(C.byref(d), C.byref(hp), C.byref(hl), info.ctypes.data_as(C.POINTER(C.c_int32)),
+                                                _dp(lines)), "clc_problems_create_from_scans")
+    return Problem(hp), Problem(hl), info, lines
+
+
+def scan_stats():
+    """Phase times (ms) and PCIe bytes of this thread's most recent problems_from_scans (clc_scan_last_stats)."""
+    ms, h2d, d2h = (C.c_float * 6)(), C.c_int64(), C.c_int64()
+    _lib.check(_lib.load().clc_scan_last_stats(ms, C.byref(h2d), C.byref(d2h)), "clc_scan_last_stats")
+    names = ("h2d", "classify", "scan", "gather", "line_fit", "finish")
+    return dict(**{k + "_ms": float(v) for k, v in zip(names, ms)}, bytes_h2d=h2d.value, bytes_d2h=d2h.value)
+
+
 def LineFittingCeres(Points, Line: np.ndarray, max_num_iterations=10):
     """reference src/LaseCamCalCeres.cpp:401-433: ``Line`` (2,) is the start value on entry and the fit on exit."""
     pts = np.ascontiguousarray(Points, dtype=np.float64).reshape(-1, 3)
@@ -510,7 +556,12 @@ def LineFittingCeres(Points, Line: np.ndarray, max_num_iterations=10):
 def CamLaserCalClosedSolution(obs, Tlc: np.ndarray, verbose=True):
     """reference src/LaseCamCalCeres.cpp:112-203.  Writes T_lc (4x4) into ``Tlc``; uses obs[i].points_on_line."""
     with Problem.from_observations(obs, use_linefitting_data=True, use_boundary_constraint=False) as p:
-        T, unobservable, _, _ = p.closed_form()
+        return closed_form_on(p, Tlc, verbose)
+
+
+def closed_form_on(p: Problem, Tlc: np.ndarray, verbose=True):
+    """CamLaserCalClosedSolution on a problem that already holds the points_on_line (e.g. from problems_from_scans)."""
+    T, unobservable, _, _ = p.closed_form()
     if unobservable and verbose:
         print("\n~~~~~~~~~~~~~~~~~~~~~~~~~~~~~~~~~~~~~~~~~~~~~~~~~~")
         print(" Notice Notice Notice: system unobservable !!!!!!!")
@@ -526,13 +577,18 @@ def CamLaserCalibration(obs, Tcl: np.ndarray, use_linefitting_data=True, use_bou
     """reference src/LaseCamCalCeres.cpp:213-383.  ``Tcl`` (4x4) is the initial guess on entry and the result on
     exit (bottom row untouched, :313-314).  Returns a dict with the solver summary and the analysis-tail outputs the
     reference prints (H singular values, null-space basis, chi2/2)."""
-    pose = T_to_pose7(Tcl)  # :215-219
     with Problem.from_observations(obs, use_linefitting_data, use_boundary_constraint) as p:
-        x, s, trace = p.solve(pose, options)
-        T = pose7_to_T(x)
-        Tcl[:3, :] = T[:3, :]  # :311-314
-        H, b, chi, sv = p.information(x)  # :318-362
-        V = p.last_V
+        return calibrate_on(p, Tcl, verbose, options)
+
+
+def calibrate_on(p: Problem, Tcl: np.ndarray, verbose=True, options: LmOptions | None = None):
+    """CamLaserCalibration on a problem that already holds the selected point set (e.g. from problems_from_scans)."""
+    pose = T_to_pose7(Tcl)  # :215-219
+    x, s, trace = p.solve(pose, options)
+    T = pose7_to_T(x)
+    Tcl[:3, :] = T[:3, :]  # :311-314
+    H, b, chi, sv = p.information(x)  # :318-362
+    V = p.last_V
     report = dict(termination=TERMINATION.get(s.termination, "?"), iterations=s.num_iterations,
                   initial_cost=s.initial_cost, final_cost=s.final_cost, trace=trace, H=H, b=b, chi2=chi / 2.0,
                   singular_values=sv, V=V, pose7=x, device_ms=s.device_ms, num_sweeps=s.num_sweeps)

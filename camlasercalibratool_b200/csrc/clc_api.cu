@@ -17,9 +17,12 @@
 #include <string>
 #include <vector>
 
+#include <cub/device/device_scan.cuh>
+
 #include "../../include/clc_b200.h"
 #include "clc_kernels.cuh"
 #include "clc_linefit.cuh"
+#include "clc_scans.cuh"
 #include "clc_small.cuh"
 
 namespace {
@@ -1476,6 +1479,208 @@ int clc_scan_segments(const float* ranges, int64_t n_scans, int64_t n_beams, dou
   cudaStreamSynchronize(st);
   cudaStreamDestroy(st);
   if (e != cudaSuccess) return fail(CLC_ERR_CUDA, cudaGetErrorString(e));
+  return CLC_OK;
+}
+
+// ---- the offline driver's scan loop on the device (clc_scans.cuh) --------------------------------------------------
+
+namespace {
+struct ScanStats {
+  float ms[6] = {};
+  int64_t bytes_h2d = 0, bytes_d2h = 0;
+};
+thread_local ScanStats g_scan_stats;
+
+// an empty problem on `device` with its stream: the caller fills the sizes and allocates
+int scan_problem_shell(clc_problem** out, const clc_scan_desc* d) {
+  clc_problem* p = new clc_problem();
+  *out = p;
+  int rc = init_device(p, d->device);
+  if (rc != CLC_OK) return rc;
+  p->use_loss = d->use_loss;
+  p->cauchy_a = d->cauchy_a;
+  // a 2-D laser: every z is 0 by construction, no z stream to scan (finish_create materialises an all-zero one only
+  // for the general kernels, below the planar size rule)
+  p->z_all_zero = true;
+  p->host_planarity_known = true;
+  return CLC_OK;
+}
+
+// the arrays of a problem of N frames and P points (as create_shell allocates them)
+int scan_problem_alloc(clc_problem* p, int64_t N, int64_t P, bool with_edges) {
+  p->n_frames = N;
+  p->n_points = P;
+  p->n_edges = with_edges ? 2 * N : 0;
+  int rc = alloc_points(p, /*with_z=*/false);
+  if (rc != CLC_OK) return rc;
+  CLC_CUDA(cudaMallocAsync(&p->frame_pose, sizeof(double) * 7 * std::max<int64_t>(N, 1), p->stream));
+  CLC_CUDA(cudaMallocAsync(&p->plane, sizeof(double) * 4 * std::max<int64_t>(N, 1), p->stream));
+  CLC_CUDA(cudaMallocAsync(&p->offsets, sizeof(int64_t) * (N + 1), p->stream));
+  CLC_CUDA(cudaMemsetAsync(p->offsets, 0, sizeof(int64_t), p->stream));
+  if (p->n_edges > 0) {
+    CLC_CUDA(cudaMallocAsync(&p->edge_plane, sizeof(double) * 4 * p->n_edges, p->stream));
+    CLC_CUDA(cudaMallocAsync(&p->edge_pt, sizeof(double) * 3 * p->n_edges, p->stream));
+  }
+  return CLC_OK;
+}
+}  // namespace
+
+int clc_problems_create_from_scans(const clc_scan_desc* d, clc_problem** points_out, clc_problem** on_line_out,
+                                   int32_t* scan_info, double* scan_line) {
+  if (points_out) *points_out = nullptr;
+  if (on_line_out) *on_line_out = nullptr;
+  if (!d) return fail(CLC_ERR_INVALID, "NULL scan description");
+  const int64_t S = d->n_scans, B = d->n_beams, K = d->n_poses;
+  if (S < 0 || B < 0 || K < 0) return fail(CLC_ERR_INVALID, "negative scan / beam / pose count");
+  if (B > INT32_MAX) return fail(CLC_ERR_INVALID, "n_beams exceeds INT32_MAX (beam indices are int32)");
+  if (S >= ((int64_t)1 << 31)) return fail(CLC_ERR_INVALID, "too many scans (frame indices are int32)");
+  if (S > 0 && B > 0 && !d->ranges) return fail(CLC_ERR_INVALID, "ranges is NULL");
+  if (S > 0 && !d->scan_stamp) return fail(CLC_ERR_INVALID, "scan_stamp is NULL");
+  if (K > 0 && (!d->pose_stamp || !d->pose_wc)) return fail(CLC_ERR_INVALID, "pose_stamp / pose_wc is NULL");
+  if (!clc::is_finite(d->angle_increment)) return fail(CLC_ERR_INVALID, "angle_increment must be finite");
+  if (!(d->max_dt > 0.0)) return fail(CLC_ERR_INVALID, "max_dt must be positive");
+  if (!(d->cauchy_a > 0.0)) return fail(CLC_ERR_INVALID, "cauchy_a must be positive");
+  if (d->line_fit_max_iterations < 0) return fail(CLC_ERR_INVALID, "line_fit_max_iterations < 0");
+
+  ScanStats st;
+  clc_problem *pa = nullptr, *pb = nullptr;
+  float* d_ranges = nullptr;
+  double *d_stamp = nullptr, *d_pose_stamp = nullptr, *d_pose_wc = nullptr, *d_lines = nullptr, *d_scan_line = nullptr;
+  int* d_info = nullptr;
+  int64_t *d_cnt = nullptr, *d_excl = nullptr;
+  void* d_tmp = nullptr;
+  cudaEvent_t ev[7] = {};
+  auto body = [&]() -> int {
+    int rc = scan_problem_shell(&pa, d);
+    if (rc != CLC_OK) return rc;
+    rc = scan_problem_shell(&pb, d);
+    if (rc != CLC_OK) return rc;
+    cudaStream_t sa = pa->stream;
+    for (cudaEvent_t& e : ev) CLC_CUDA(cudaEventCreate(&e));
+    // -- H2D: the ranges (4 B per beam), the stamps and the poses; nothing else crosses PCIe towards the device
+    CLC_CUDA(cudaEventRecord(ev[0], sa));
+    const size_t range_bytes = sizeof(float) * (size_t)S * (size_t)B;
+    CLC_CUDA(cudaMallocAsync(&d_ranges, std::max<size_t>(range_bytes, 4), sa));
+    CLC_CUDA(cudaMallocAsync(&d_stamp, sizeof(double) * std::max<int64_t>(S, 1), sa));
+    CLC_CUDA(cudaMallocAsync(&d_pose_stamp, sizeof(double) * std::max<int64_t>(K, 1), sa));
+    CLC_CUDA(cudaMallocAsync(&d_pose_wc, sizeof(double) * 7 * std::max<int64_t>(K, 1), sa));
+    CLC_CUDA(cudaMallocAsync(&d_info, sizeof(int) * 4 * std::max<int64_t>(S, 1), sa));
+    CLC_CUDA(cudaMallocAsync(&d_cnt, sizeof(int64_t) * 2 * (S + 1), sa));
+    CLC_CUDA(cudaMallocAsync(&d_excl, sizeof(int64_t) * 2 * (S + 1), sa));
+    if (range_bytes > 0) CLC_CUDA(cudaMemcpyAsync(d_ranges, d->ranges, range_bytes, cudaMemcpyHostToDevice, sa));
+    if (S > 0) CLC_CUDA(cudaMemcpyAsync(d_stamp, d->scan_stamp, sizeof(double) * S, cudaMemcpyHostToDevice, sa));
+    if (K > 0) {
+      CLC_CUDA(cudaMemcpyAsync(d_pose_stamp, d->pose_stamp, sizeof(double) * K, cudaMemcpyHostToDevice, sa));
+      CLC_CUDA(cudaMemcpyAsync(d_pose_wc, d->pose_wc, sizeof(double) * 7 * K, cudaMemcpyHostToDevice, sa));
+    }
+    st.bytes_h2d = (int64_t)range_bytes + 8 * S + 8 * K + 56 * K;
+    CLC_CUDA(cudaEventRecord(ev[1], sa));
+    // -- classify: segment + nearest pose per scan
+    CLC_CUDA(cudaMemsetAsync(d_excl, 0, sizeof(int64_t) * 2 * (S + 1), sa));
+    if (S > 0) {
+      clc::clc_scan_classify_kernel<<<(unsigned)((S + clc::kClassifyThreads) / clc::kClassifyThreads), clc::kClassifyThreads, 0, sa>>>(
+          d_ranges, S, B, d->angle_min, d->angle_increment, d->range_min, d_stamp, d_pose_stamp, K, d->max_dt, d_info, d_cnt);
+      CLC_LAUNCH_CHECK();
+    }
+    CLC_CUDA(cudaEventRecord(ev[2], sa));
+    // -- exclusive scans (integer: deterministic) -> frame index per scan, point offset per scan; the totals at [S]
+    int64_t totals[2] = {0, 0};
+    if (S > 0) {
+      size_t tmp_bytes = 0;
+      CLC_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, d_cnt, d_excl, S + 1, sa));
+      CLC_CUDA(cudaMallocAsync(&d_tmp, tmp_bytes, sa));
+      CLC_CUDA(cub::DeviceScan::ExclusiveSum(d_tmp, tmp_bytes, d_cnt, d_excl, S + 1, sa));
+      CLC_CUDA(cub::DeviceScan::ExclusiveSum(d_tmp, tmp_bytes, d_cnt + S + 1, d_excl + S + 1, S + 1, sa));
+      g_launches.fetch_add(2);
+      CLC_CUDA(cudaMemcpyAsync(&totals[0], d_excl + S, sizeof(int64_t), cudaMemcpyDeviceToHost, sa));
+      CLC_CUDA(cudaMemcpyAsync(&totals[1], d_excl + 2 * S + 1, sizeof(int64_t), cudaMemcpyDeviceToHost, sa));
+    }
+    CLC_CUDA(cudaEventRecord(ev[3], sa));
+    CLC_CUDA(cudaStreamSynchronize(sa));  // the only host sync before the allocations
+    st.bytes_d2h = S > 0 ? 16 : 0;
+    const int64_t F = totals[0], P = totals[1];
+    // -- allocate both problems, gather the points problem
+    rc = scan_problem_alloc(pa, F, P, false);
+    if (rc != CLC_OK) return rc;
+    rc = scan_problem_alloc(pb, F, 2 * F, d->with_edges != 0);
+    if (rc != CLC_OK) return rc;
+    CLC_CUDA(cudaStreamSynchronize(pb->stream));  // pb's arrays are written on sa below
+    if (S > 0) {
+      const int warps = 8;
+      clc::clc_scan_gather_kernel<<<(unsigned)((S + warps - 1) / warps), warps * 32, 0, sa>>>(
+          d_ranges, S, B, d->angle_min, d->angle_increment, d->range_min, d_pose_wc, d_cnt, d_excl, d_info, pa->x, pa->y,
+          pa->frame_pose, pa->offsets);
+      CLC_LAUNCH_CHECK();
+    }
+    CLC_CUDA(cudaFreeAsync(d_ranges, sa));  // the largest buffer goes back to the pool before the line fit
+    d_ranges = nullptr;
+    CLC_CUDA(cudaEventRecord(ev[4], sa));
+    // -- batched LineFittingCeres from a zero start (calibr_offline.cpp:123-124; CauchyLoss(0.05), LaseCamCalCeres.cpp:416),
+    //    then the on-line problem device to device
+    CLC_CUDA(cudaMallocAsync(&d_lines, sizeof(double) * 2 * std::max<int64_t>(F, 1), sa));
+    if (F > 0) {
+      CLC_CUDA(cudaMemsetAsync(d_lines, 0, sizeof(double) * 2 * F, sa));
+      const int warps = 8;
+      clc::clc_line_fit_kernel<<<(unsigned)((F + warps - 1) / warps), warps * 32, 0, sa>>>(
+          pa->x, pa->y, pa->offsets, F, d->line_fit_max_iterations, 0.05, d_lines, nullptr);
+      CLC_LAUNCH_CHECK();
+      clc::clc_scan_on_line_kernel<<<(unsigned)((F + 255) / 256), 256, 0, sa>>>(pa->x, pa->y, pa->offsets, pa->frame_pose, d_lines, F,
+                                                                               pb->x, pb->y, pb->frame_pose, pb->offsets, pb->edge_pt);
+      CLC_LAUNCH_CHECK();
+    }
+    if (scan_line && S > 0) {
+      CLC_CUDA(cudaMallocAsync(&d_scan_line, sizeof(double) * 2 * S, sa));
+      clc::clc_scan_lines_kernel<<<(unsigned)((S + 255) / 256), 256, 0, sa>>>(d_info, S, d_lines, d_scan_line);
+      CLC_LAUNCH_CHECK();
+      CLC_CUDA(cudaMemcpyAsync(scan_line, d_scan_line, sizeof(double) * 2 * S, cudaMemcpyDeviceToHost, sa));
+      st.bytes_d2h += 16 * S;
+    }
+    if (scan_info && S > 0) {
+      CLC_CUDA(cudaMemcpyAsync(scan_info, d_info, sizeof(int) * 4 * S, cudaMemcpyDeviceToHost, sa));
+      st.bytes_d2h += 16 * S;
+    }
+    CLC_CUDA(cudaEventRecord(ev[5], sa));
+    // -- planes, partition (finish_create synchronises each problem's stream: pb's inputs were written on sa, which is
+    //    complete once finish_create(pa) returns)
+    rc = finish_create(pa);
+    if (rc != CLC_OK) return rc;
+    rc = finish_create(pb);
+    if (rc != CLC_OK) return rc;
+    CLC_CUDA(cudaEventRecord(ev[6], pb->stream));
+    CLC_CUDA(cudaEventSynchronize(ev[6]));
+    for (int i = 0; i < 6; ++i) CLC_CUDA(cudaEventElapsedTime(&st.ms[i], ev[i], ev[i + 1]));
+    return CLC_OK;
+  };
+  int rc = body();
+  if (pa && pa->stream) {
+    void* bufs[] = {d_ranges, d_stamp, d_pose_stamp, d_pose_wc, d_lines, d_scan_line, d_info, d_cnt, d_excl, d_tmp};
+    for (void* b : bufs)
+      if (b) cudaFreeAsync(b, pa->stream);
+  }
+  for (cudaEvent_t e : ev)
+    if (e) cudaEventDestroy(e);
+  if (rc == CLC_OK && pa && pa->stream) {
+    cudaError_t e = cudaStreamSynchronize(pa->stream);
+    if (e != cudaSuccess) rc = fail(CLC_ERR_CUDA, cudaGetErrorString(e));
+  }
+  if (rc != CLC_OK) {
+    const std::string msg = g_last_error;
+    clc_problem_destroy(pa);
+    clc_problem_destroy(pb);
+    g_last_error = msg;
+    return rc;
+  }
+  g_scan_stats = st;
+  if (points_out) *points_out = pa; else clc_problem_destroy(pa);
+  if (on_line_out) *on_line_out = pb; else clc_problem_destroy(pb);
+  return CLC_OK;
+}
+
+int clc_scan_last_stats(float phase_ms6[6], int64_t* bytes_h2d, int64_t* bytes_d2h) {
+  if (phase_ms6)
+    for (int i = 0; i < 6; ++i) phase_ms6[i] = g_scan_stats.ms[i];
+  if (bytes_h2d) *bytes_h2d = g_scan_stats.bytes_h2d;
+  if (bytes_d2h) *bytes_d2h = g_scan_stats.bytes_d2h;
   return CLC_OK;
 }
 

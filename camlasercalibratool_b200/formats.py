@@ -9,6 +9,8 @@ closed form, LM solve, information matrix -- goes through the CUDA library.
   -- reference main/calibr_offline.cpp:186-197.
 * ``calibrate_offline``  reference main/calibr_offline.cpp:52-170 from key-frame thinning to the LM solve, taking the
   already-extracted laser segments (the output of AutoGetLinePts) instead of a rosbag.
+* ``calibrate_offline_from_scans``  the same from the raw LaserScan ranges: the scan loop (segment, nearest pose, line fit,
+  end points) runs on the device and builds both problems there (clc_problems_create_from_scans).
 """
 from __future__ import annotations
 
@@ -281,5 +283,35 @@ def calibrate_offline(tagpose, scans, result_yaml=None, verbose=False):
     if result_yaml is not None:
         write_result_yaml(result_yaml, Tlc)
     report["n_obs"] = len(obs)
+    report["Tlc_closed_form"] = Tlc0
+    return Tlc, report
+
+
+def calibrate_offline_from_scans(tagpose, scan_stamps, ranges, angle_min, angle_increment, range_min, result_yaml=None,
+                                 verbose=False):
+    """reference main/calibr_offline.cpp:52-197 from the raw LaserScan ranges[n_scans, n_beams] (float32) and their stamps:
+    the same result as ``calibrate_offline(tagpose, segments_from_scans(scan_stamps, ranges, ...))``, but the scan loop
+    (segment, nearest key-frame pose, line fit, end points) runs on the device and the points never leave it -- one upload
+    of the ranges.  Key-frame thinning stays on the host (sequential, O(poses)).  Returns (Tlc, report) or (None, reason)."""
+    from .api import calibrate_on, closed_form_on, problems_from_scans
+
+    if len(tagpose) < 10:  # :55-59
+        return None, "apriltag pose less than 10."
+    kf = select_keyframes(tagpose)
+    stamps = np.array([p.timestamp for p in kf], dtype=np.float64)
+    pose_wc = np.array([np.concatenate([p.qwc, p.twc]) for p in kf], dtype=np.float64).reshape(-1, 7)
+    points, on_line, _, _ = problems_from_scans(ranges, scan_stamps, angle_min, angle_increment, range_min, stamps, pose_wc)
+    with points, on_line:
+        n_obs = points.sizes()[0]
+        if n_obs < 5:  # :158-163
+            return None, "Valid Calibra Data Less"
+        Tlc0 = np.eye(4)
+        closed_form_on(on_line, Tlc0, verbose=verbose)  # :166-167
+        Tcl = np.linalg.inv(Tlc0)
+        report = calibrate_on(points, Tcl, verbose=verbose)  # :169-170
+    Tlc = np.linalg.inv(Tcl)
+    if result_yaml is not None:
+        write_result_yaml(result_yaml, Tlc)
+    report["n_obs"] = n_obs
     report["Tlc_closed_form"] = Tlc0
     return Tlc, report

@@ -211,6 +211,39 @@ int clc_line_fit_points(const double* points_xyz, int64_t n, double line[2], int
 int clc_scan_segments(const float* ranges, int64_t n_scans, int64_t n_beams, double angle_min, double angle_increment,
                       double range_min, int32_t* seg_start, int32_t* seg_end, int device);
 
+/* replaces: the scan loop of the offline driver, reference main/calibr_offline.cpp:86-155 -- TranScanToPoints
+ * (src/utilities.cpp:181-215), AutoGetLinePts (src/selectScanPoints.cpp:17-190), the nearest tag pose (:103-116),
+ * LineFittingCeres (src/LaseCamCalCeres.cpp:385-433), the line end points (:126-142) and the Oberserve it fills (:144-150)
+ * -- for a whole batch of LaserScans, on the device.  Only the ranges, the stamps and the poses cross PCIe; the two problems
+ * the driver then solves are built device to device:
+ *   *points  : Oberserve::points of every frame (CamLaserCalibration(obs, Tcl, false), :170), no edge residuals;
+ *   *on_line : Oberserve::points_on_line, two per frame (CamLaserCalClosedSolution, :167), with the board-edge residuals
+ *              (front and back of obs.points) when with_edges.
+ * A frame is a scan with a board segment whose nearest pose (linear search: strict <, ties to the lowest index, NaN stamps
+ * never match, poses in any order) lies strictly within max_dt; frames keep scan order.  frame_pose = (qwc^-1, -R(qwc^-1) twc)
+ * with Eigen semantics (no normalisation).  Points are the beams seg_start..seg_end of the scan (invalid beams inside a
+ * segment included as (1000, 1000), as the reference keeps them), z = 0.  The lines are fitted from a zero start with
+ * CauchyLoss(0.05).  Both problems are planar by construction.  Either output may be NULL; on failure both are NULL.
+ * scan_info[n_scans*4] (optional) = seg_start, seg_end, nearest pose (-1: no segment or no pose), frame (-1: not kept);
+ * scan_line[n_scans*2] (optional) = the fitted line of a kept scan, NaN otherwise.  Bit-reproducible. */
+typedef struct {
+  int64_t n_scans, n_beams;
+  const float* ranges;          /* host [n_scans*n_beams], LaserScan::ranges row by row; pinned memory is the DMA source */
+  const double* scan_stamp;     /* host [n_scans], header.stamp.toSec() */
+  double angle_min, angle_increment, range_min; /* the LaserScan fields */
+  int64_t n_poses;
+  const double* pose_stamp;     /* host [n_poses] */
+  const double* pose_wc;        /* host [n_poses*7] qx qy qz qw x y z of T_wc (the layout of clc_estimate_board_poses) */
+  double max_dt;                /* 0.02 s in the reference (:116) */
+  int line_fit_max_iterations;  /* 10 */
+  int with_edges;               /* board-edge residuals on the on-line problem (use_boundary_constraint) */
+  int use_loss;
+  double cauchy_a;
+  int device;
+} clc_scan_desc;
+int clc_problems_create_from_scans(const clc_scan_desc* d, clc_problem** points, clc_problem** on_line, int32_t* scan_info,
+                                   double* scan_line);
+
 /* Board poses from detected tag corners, batched: the arithmetic of CamPoseEst::calcCamPose after the tag detector
  * (reference src/calcCamPose.cpp:270-294: liftProjective of every corner, x/z y/z as cv::Point2f) and of
  * CamPoseEst::EstimatePose (:211-236: solvePnP with identity intrinsics on the kalibr-grid object points :114-136,
@@ -307,6 +340,9 @@ int clc_upload_last_stats(double* total_ms, double* pack_wait_ms, int64_t* bytes
  * pairs (xy != 0; *nonplanar = a z != 0 or NaN was met) or packed x,y,z. */
 int clc_debug_pack(int64_t n_frames, const double* const* frame_points, const int64_t* frame_counts, int64_t a, int64_t b,
                    int xy, double* out, int* nonplanar);
+/* Phase times (CUDA events, ms) of this thread's most recent clc_problems_create_from_scans: H2D, classify, scan (+ the
+ * D2H of the totals), gather (+ allocation), line fit (+ on-line build), finish; and the bytes it moved H2D / D2H. */
+int clc_scan_last_stats(float phase_ms6[6], int64_t* bytes_h2d, int64_t* bytes_d2h);
 /* Raw PCIe yardstick: `reps` host(pinned) -> device copies of `bytes` on `device`, each timed with CUDA events. */
 int clc_bench_h2d(int64_t bytes, int device, int reps, float* ms_each);
 /* Bytes clc_solve_lm reads back per solve (LM state + iteration trace). */
